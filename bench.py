@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py - Msamples/s of the Mode S receive hot path (IQ demod + preamble detect + slice + CRC).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--log2n 28]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--log2n 28] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (BASELINE.json configs[1]): synthetic 1090 MHz IQ at 4 Msps, 2^28 complex samples (2 GiB) per GPU,
@@ -14,6 +14,9 @@ same size (weak scaling, no data-path collective; NCCL only fans the buffers out
   roofline     scan kernel: 8 algorithmic bytes/sample / its measured duration vs the measured HBM peak
   cpu_baseline the reference's own C++ (oracle/_ref: unmodified preamble_impl/slicer_impl/modes_crc behind the
                restated GNU Radio front end) on a bounded sample, all host threads
+
+--dump-outputs DIR writes the frames the headline's last timed step delivered (see dump_outputs). The input is seeded,
+so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -34,6 +37,7 @@ RATE = 4e6
 THRESHOLD_DB = 7.0
 N_BURSTS = 1000
 NOISE_SIGMA = 0.01
+DUMP_LIMIT_BYTES = 64 << 20
 
 
 def measured_peak_gbs():
@@ -180,7 +184,22 @@ def parity_check(rx, q, iq, rate, threads):
             "detections": d, "oracle": kind, "seconds": round(time.perf_counter() - t0, 1)}
 
 
-def run_config(key, n, args, rank, local_rank, world, device, fan=None, steps=None):
+def dump_outputs(out_dir, frames):
+    """What a caller of the timed path receives: its frames (struct amb_frame, stream order), one float64 array per
+    field as out_dir/<field>.npy; lowconfbits and data are [n, 24] and [n, 14]. Beyond DUMP_LIMIT_BYTES in all, a fixed
+    seeded sample of the frames (kept in stream order) is written instead."""
+    from gr_air_modes_b200._lib import Frame
+    rec = np.frombuffer(b"".join(bytes(f) for f in frames), dtype=np.dtype(Frame))
+    names = [name for name, _ in Frame._fields_ if name != "pad_"]
+    per_frame = 8 * sum(int(np.prod(rec.dtype[name].shape)) for name in names)
+    if rec.size * per_frame > DUMP_LIMIT_BYTES:
+        rec = rec[np.sort(np.random.default_rng(0).choice(rec.size, DUMP_LIMIT_BYTES // per_frame, replace=False))]
+    os.makedirs(out_dir, exist_ok=True)
+    for name in names:
+        np.save(os.path.join(out_dir, name + ".npy"), rec[name].astype(np.float64))
+
+
+def run_config(key, n, args, rank, local_rank, world, device, fan=None, steps=None, dump_dir=None):
     """Device-resident timing + full-size parity of one BASELINE config. Returns (result dict, iq, rx, q)."""
     import torch
     import torch.distributed as dist
@@ -224,7 +243,10 @@ def run_config(key, n, args, rank, local_rank, world, device, fan=None, steps=No
     scan_ms = rx._ctx.scan_times_ms(min(steps, 64))
     st = rx.stats()
     launches = st.kernel_launches - launches0
-    rx.drain(); q.flush()
+    rx.drain()                     # the last timed step's frames: reset() dropped the earlier steps' results
+    if dump_dir:
+        dump_outputs(dump_dir, rx.frames)
+    q.flush()
     ms_max = shard.max_over_ranks(ms, world, device)
     scan_avg = shard.max_over_ranks(float(np.mean(scan_ms)), world, device)
     peak, peak_src = measured_peak_gbs()
@@ -609,6 +631,8 @@ def main():
     ap.add_argument("--no-parity", action="store_true")
     ap.add_argument("--no-e2e-extras", action="store_true")
     ap.add_argument("--no-e2e", action="store_true", help="profiling runs only: skip the end-to-end legs (the line then has no e2e)")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR", help="write the frames of the headline's last timed "
+                    "step as DIR/<field>.npy (rank 0)")
     ap.add_argument("--time-shard", action="store_true",
                     help="secondary mode: ONE 2^log2n-sample recording cut into --gpus spans (strong scaling)")
     ap.add_argument("--chain", action="store_true", help="--time-shard: plain hand-over chain instead of speculative resolution")
@@ -661,7 +685,8 @@ def main():
     if rank == 0:
         sampler.start()
     all_cpus = os.sched_getaffinity(0)
-    head, iq, rx, q = run_config(key, n, args, rank, local_rank, world, device)
+    head, iq, rx, q = run_config(key, n, args, rank, local_rank, world, device,
+                                 dump_dir=args.dump_outputs if rank == 0 else None)
     e2e, e2e_extras = (None, {}) if args.no_e2e else e2e_legs(rx, q, iq, n, args, local_rank, world, device)
     clocks = sampler.stop() if rank == 0 else None     # sampled across the headline's timed regions (device + end to end)
     os.sched_setaffinity(0, all_cpus)                  # the CPU legs below get every host thread back

@@ -27,7 +27,13 @@ def port():
 
 @pytest.fixture(scope="session")
 def ref():
-    from oracle import cpu_oracle
-    if not cpu_oracle.ref_available():
-        pytest.skip("oracle/_ref not built and /root/reference absent")
-    return cpu_oracle.Ref()
+    """The unmodified reference objects, replayed from tests/golden/ref_results.json.xz. With AMB_TEST_RECORD_REF=1
+    (tests/golden/make_ref_golden.py) the live objects answer instead and the session's calls are recorded."""
+    from helpers import RecordedRef
+    if os.environ.get("AMB_TEST_RECORD_REF") == "1":
+        from oracle import cpu_oracle
+        rec = RecordedRef(cpu_oracle.Ref())
+        yield rec
+        rec.save()
+    else:
+        yield RecordedRef()

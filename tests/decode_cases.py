@@ -213,6 +213,49 @@ def message_strings(msgs):
     return ["%s %06x %r %d %r" % (h, e, 10.0 ** (-((7 * k) % 61) / 10.0), s, f) for k, (h, e, s, f) in enumerate(msgs)]
 
 
+def fuzz_messages(n=12000, seed=77):
+    """Unconstrained message bytes (raw_message), arrival gaps exponential with a rare 12 s silence."""
+    rng = np.random.default_rng(seed)
+    msgs, t = [], 0.0
+    for _ in range(n):
+        frame, ecc = raw_message(rng)
+        t += float(rng.exponential(0.02)) + (12.0 if rng.random() < 0.001 else 0.0)
+        msgs.append((frame.hex(), ecc, int(t), t - int(t)))
+    return msgs
+
+
+FUZZ_LOCATIONS = ([37.4, -122.1], None, [-45.0, 170.0])
+
+
+def fuzz_sample(n, k=1500, seed=78):
+    """The fixed indices of fuzz_messages() whose reference results are stored (all of them would exceed 500 kB)."""
+    return sorted(int(x) for x in np.random.default_rng(seed).choice(n, k, replace=False))
+
+
+def cpr_class_script(rounds=1500):
+    """The reference's cpr.py self-test procedure (cpr.py:264-331: sweep of positions, even then odd report) plus
+    surface reports, expiry and a moving receiver location, for a cpr_decoder class on an injected clock.
+    -> {surface: (first location, [("loc", [lat, lon]) | ("decode", now, icao, lat_cpr, lon_cpr, odd), ...])}"""
+    out = {}
+    for surface in (0, 1):
+        ev = []
+        for i in range(rounds):
+            lat = i / (rounds / 170.) - 85 if not surface else 35.0 + (i % 50) * 1e-3
+            if not surface and 100 <= i < 160:
+                lat = 10.4704713 - 7e-4 + (i - 100) * 2.5e-5          # across an NL transition: boundary straddles
+            lon = i / (rounds / 360.) - 180 if not surface else -100.0 + (i % 70) * 1e-3
+            icao = (i * 7919) & 0xFFFFFF
+            now = 1000.0 + i * 0.37 + (30.0 if i == 700 else 0.0)
+            if i == 900:
+                ev.append(("loc", [34.5, -99.5]))
+            for odd, dl in ((0, 0.0), (1, 1e-3)):
+                la, lo = cpr_encode(lat + dl, min(lon + dl, 180), odd, bool(surface))
+                now += 0.01
+                ev.append(("decode", now, icao, la, lo, odd))
+        out[surface] = ([35.0, -100.0], ev)
+    return out
+
+
 CASES = [
     dict(seed=11, location=(37.4, -122.1)),
     dict(seed=12, location=None),

@@ -1,9 +1,101 @@
+import fcntl
+import hashlib
 import json
+import lzma
 import os
+import tempfile
 
 import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
+REF_RESULTS = os.path.join(HERE, "golden", "ref_results.json.xz")
+
+
+def chips_digest(chips):
+    """SHA-256 of 240-chip packets (float32), every NaN in one canonical form: equal digests = np.array_equal(equal_nan)."""
+    a = np.array(chips, dtype=np.float32)
+    a[np.isnan(a)] = np.nan
+    return hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()
+
+
+class RecordedRef:
+    """The unmodified reference objects (oracle/_ref: preamble_impl.cc, slicer_impl.cc, modes_crc.cc) as the tests see
+    them, replayed from tests/golden/ref_results.json.xz: every call the tests make is keyed by a hash of its arguments,
+    so an input the reference was never shown has no answer and the test fails. Results carry the chip packets as
+    `chips_sha256` (see chips_digest). tests/golden/make_ref_golden.py records the file by running the tests against
+    the live objects (`live`), where the reference sources exist."""
+
+    def __init__(self, live=None):
+        self.live, self.new = live, {}
+        if live is None:
+            with lzma.open(REF_RESULTS, "rt") as f:
+                self.table = json.load(f)
+
+    @staticmethod
+    def _key(name, *args):
+        h = hashlib.sha256(name.encode())
+        for a in args:
+            if isinstance(a, np.ndarray):
+                h.update(b"a" + str(a.dtype).encode() + np.ascontiguousarray(a).tobytes())
+            else:
+                h.update(b"s" + repr(a).encode())
+        return h.hexdigest()
+
+    def _call(self, key, compute):
+        if self.live is None:
+            if key not in self.table:
+                raise KeyError("no recorded reference result for this input: rerun tests/golden/make_ref_golden.py")
+            return self.table[key]
+        self.new[key] = compute()
+        return self.new[key]
+
+    def save(self):
+        """Record mode: merge this session's calls into the file (several pytest processes may record at once)."""
+        if self.live is None or not self.new:
+            return
+        with open(os.path.join(tempfile.gettempdir(), "amb_ref_results.lock"), "w") as lock:
+            fcntl.flock(lock, fcntl.LOCK_EX)
+            table = {}
+            if os.path.exists(REF_RESULTS):
+                with lzma.open(REF_RESULTS, "rt") as f:
+                    table = json.load(f)
+            table.update(self.new)
+            with lzma.open(REF_RESULTS, "wb", preset=9) as f:
+                f.write(json.dumps(table, sort_keys=True, separators=(",", ":")).encode())
+
+    @staticmethod
+    def _result(d):
+        from oracle.cpu_oracle import Result
+        r = Result(np.array(d["index"], np.uint64), np.array(d["secs"], np.uint64), np.array(d["frac"], np.float64),
+                   None, d["msgs"], None, d["calls"])
+        r.chips_sha256 = d["chips_sha256"]
+        return r
+
+    @staticmethod
+    def _record(r):
+        return {"index": [int(x) for x in r.index], "secs": [int(x) for x in r.secs], "frac": [float(x) for x in r.frac],
+                "chips_sha256": chips_digest(r.chips), "msgs": r.msgs, "calls": r.calls}
+
+    def crc24(self, data: bytes) -> int:
+        data = bytes(data)
+        return self._call(self._key("crc24", data), lambda: self.live.crc24(data))
+
+    def preamble_params(self, rate, threshold_db):
+        rate, thr = float(rate), float(threshold_db)
+        return tuple(self._call(self._key("preamble_params", rate, thr), lambda: list(self.live.preamble_params(rate, thr))))
+
+    def run_streams(self, bb, avg, rate, threshold_db, slice_=True, start_time=None):
+        bb, avg = np.ascontiguousarray(bb, np.float32), np.ascontiguousarray(avg, np.float32)
+        rate, thr = float(rate), float(threshold_db)
+        st = None if start_time is None else (int(start_time[0]), float(start_time[1]))
+        key = self._key("run_streams", bb, avg, rate, thr, bool(slice_), st)
+        return self._result(self._call(key, lambda: self._record(self.live.run_streams(bb, avg, rate, thr, slice_, st))))
+
+    def run_slicer(self, chips, secs, frac):
+        chips = np.ascontiguousarray(chips, np.float32)
+        secs, frac = np.ascontiguousarray(secs, np.uint64), np.ascontiguousarray(frac, np.float64)
+        key = self._key("run_slicer", chips, secs, frac)
+        return self._result(self._call(key, lambda: self._record(self.live.run_slicer(chips, secs, frac))))
 
 
 def load_golden():
@@ -45,6 +137,12 @@ def load_decode_golden():
     import gzip
     with gzip.open(os.path.join(HERE, "golden", "decode_golden.json.gz"), "rt") as f:
         return json.load(f)["cases"]
+
+
+def load_decode_ref_golden():
+    """What the unmodified reference modules computed for the inputs of tests/golden/make_decode_ref_golden.py."""
+    with lzma.open(os.path.join(HERE, "golden", "decode_ref_golden.json.xz"), "rt") as f:
+        return json.load(f)
 
 
 def compare_decode(rec, ref, tol=0.0, where="", tol_libm=None):

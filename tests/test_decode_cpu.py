@@ -2,7 +2,8 @@
 
   * oracle/decode_oracle.py against the committed golden produced by the UNMODIFIED reference modules
     (tests/golden/make_decode_golden.py), bit-exact incl. every float;
-  * the same against the live reference where /root/reference exists;
+  * the same on further seeds and unconstrained message bytes, against what the reference computed for them
+    (tests/golden/make_decode_ref_golden.py);
   * the product's per-message device code (gr_air_modes_b200/csrc/amb_decode_core.h, the `__host__ __device__`
     functions the CUDA kernels call) compiled for the host by tests/decode_host_shim.cc - a test-only harness, not a
     product path - against the golden, so the decode arithmetic is checked even where no GPU is present.
@@ -12,7 +13,7 @@ import sys
 
 import pytest
 
-from helpers import compare_decode, load_decode_golden
+from helpers import compare_decode, load_decode_golden, load_decode_ref_golden
 
 sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
 
@@ -29,23 +30,16 @@ def test_decode_oracle_matches_reference_golden():
     assert n > 5000
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/python"), reason="reference tree not present")
 def test_decode_oracle_matches_live_reference_on_fresh_seeds():
     import decode_cases
     from oracle import decode_oracle as do
-    sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden"))
-    import make_decode_golden as mg
-    mods = mg.load_reference()
-    try:
-        for seed in (101, 102, 103):
-            loc, msgs = decode_cases.make_case(seed, location=(None if seed == 102 else (40.0 + seed % 7, -70.0)),
-                                               seconds=30.0, surface_share=0.4)
-            ref = mg.run_reference(loc, msgs, mods)
-            recs = do.decode_batch(msgs, loc)
-            for k, (rec, r) in enumerate(zip(recs, ref)):
-                compare_decode(rec, r, 0.0, "seed %d msg %d" % (seed, k))
-    finally:
-        mg.unload_reference()
+    for case in load_decode_ref_golden()["fresh"]:
+        seed = case["seed"]
+        loc, msgs = decode_cases.make_case(seed, location=case["location"], seconds=30.0, surface_share=0.4)
+        recs = do.decode_batch(msgs, loc)
+        assert len(recs) == len(case["ref"])
+        for k, (rec, r) in enumerate(zip(recs, case["ref"])):
+            compare_decode(rec, r, 0.0, "seed %d msg %d" % (seed, k))
 
 
 # ---- the product's decode arithmetic, compiled for the host by a test-only shim -------------------------------------
@@ -152,38 +146,28 @@ def test_report_lines_match_reference_printer(shim):
     assert n > 5000 and printed > 4000
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/python"), reason="reference tree not present")
 def test_fuzz_oracle_core_and_reports_against_live_reference(shim):
     """Unconstrained message bytes (incl. what no slicer emits: long DFs in 56 bits, short DFs in 112 bits) through
     the UNMODIFIED parse.py / altitude.py / cpr.py / msprint.py, the oracle, the host build of the product's decode
-    arithmetic, and report.py: all four agree message by message."""
-    import numpy as np
+    arithmetic, and report.py: all four agree message by message. The whole stream is decoded (CPR state carries
+    across messages); the reference's results are stored for a fixed sample of 1500 of its 12000 messages."""
     import decode_cases
     from gr_air_modes_b200 import report
     from oracle import decode_oracle as do
-    sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden"))
-    import make_decode_golden as mg
-    mods = mg.load_reference()
-    try:
-        rng = np.random.default_rng(77)
-        msgs, t = [], 0.0
-        for _ in range(12000):
-            frame, ecc = decode_cases.raw_message(rng)
-            t += float(rng.exponential(0.02)) + (12.0 if rng.random() < 0.001 else 0.0)
-            msgs.append((frame.hex(), ecc, int(t), t - int(t)))
-        texts = decode_cases.message_strings(msgs)
-        for loc in ([37.4, -122.1], None, [-45.0, 170.0]):
-            ref = mg.run_reference(loc, msgs, mods)
-            lines = mg.run_reference_printer(loc, msgs, mods)
-            want = do.decode_batch(msgs, loc)
-            got = _shim_decode(shim, msgs, loc)
-            for k, (w, g, r, text, line) in enumerate(zip(want, got, ref, texts, lines)):
-                compare_decode(w, r, 0.0, "oracle %d %s" % (k, msgs[k][0]))
-                compare_decode(g, r, 0.0, "core %d %s" % (k, msgs[k][0]), tol_libm=1e-13)
-                assert report.format_report(text, g) == line, (k, text)
-            assert sum("pos" in r for r in ref) > 300
-    finally:
-        mg.unload_reference()
+    msgs = decode_cases.fuzz_messages()
+    keep = decode_cases.fuzz_sample(len(msgs))
+    texts = decode_cases.message_strings(msgs)
+    stored = load_decode_ref_golden()["fuzz"]
+    assert [c["location"] for c in stored] == list(decode_cases.FUZZ_LOCATIONS)
+    for case in stored:
+        loc = case["location"]
+        want = do.decode_batch(msgs, loc)
+        got = _shim_decode(shim, msgs, loc)
+        for k, r, line in zip(keep, case["ref"], case["lines"]):
+            compare_decode(want[k], r, 0.0, "oracle %d %s" % (k, msgs[k][0]))
+            compare_decode(got[k], r, 0.0, "core %d %s" % (k, msgs[k][0]), tol_libm=1e-13)
+            assert report.format_report(texts[k], got[k]) == line, (k, texts[k])
+        assert sum("pos" in r for r in case["ref"]) > 40
 
 
 class _ShimBackend:
@@ -209,59 +193,41 @@ class _ShimBackend:
         return out
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/python"), reason="reference tree not present")
 def test_cpr_decoder_dropin_class_against_the_reference_class(shim):
-    """decode.cpr_decoder (same methods, return list and exceptions as python/cpr.py:183-240) side by side with the
-    UNMODIFIED reference class on the reference's own self-test procedure (cpr.py:264-331: sweep of positions, even
-    then odd report) plus surface reports, expiry and a moving receiver location; both run on one injected clock."""
+    """decode.cpr_decoder (same methods, return list and exceptions as python/cpr.py:183-240) against what the
+    UNMODIFIED reference class returned on the reference's own self-test procedure (cpr.py:264-331: sweep of
+    positions, even then odd report) plus surface reports, expiry and a moving receiver location, on one injected
+    clock (decode_cases.cpr_class_script)."""
     import decode_cases as dc
     from gr_air_modes_b200 import decode
     from gr_air_modes_b200.errors import CPRBoundaryStraddleError, CPRNoPositionError
     sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden"))
     import make_decode_golden as mg
-    exc, alt, parse, cpr = mg.load_reference()
-    try:
-        clock = mg.Clock()
-        cpr.time = type("T", (), {"time": staticmethod(clock.time)})
-        rounds, ok, straddle, nopos = 1500, 0, 0, 0
-        for surface in (0, 1):
-            loc = [35.0, -100.0]
-            ref = cpr.cpr_decoder(list(loc))
-            ours = decode.cpr_decoder(list(loc), clock=clock.time, _backend=_ShimBackend(shim, list(loc)))
-            for i in range(rounds):
-                lat = i / (rounds / 170.) - 85 if not surface else 35.0 + (i % 50) * 1e-3
-                if not surface and 100 <= i < 160:
-                    lat = 10.4704713 - 7e-4 + (i - 100) * 2.5e-5          # across an NL transition: boundary straddles
-                lon = i / (rounds / 360.) - 180 if not surface else -100.0 + (i % 70) * 1e-3
-                icao = (i * 7919) & 0xFFFFFF
-                clock.now = 1000.0 + i * 0.37 + (30.0 if i == 700 else 0.0)
-                if i == 900:
-                    loc = [34.5, -99.5]
-                    ref.set_location(list(loc)); ours.set_location(list(loc))
-                for odd, dl in ((0, 0.0), (1, 1e-3)):
-                    la, lo = dc.cpr_encode(lat + dl, min(lon + dl, 180), odd, bool(surface))
-                    clock.now += 0.01
-                    want = got = None
-                    try:
-                        want = ref.decode(icao, la, lo, odd, surface)
-                    except exc.CPRBoundaryStraddleError:
-                        want = "straddle"
-                    except exc.CPRNoPositionError:
-                        want = "nopos"
-                    try:
-                        got = ours.decode(icao, la, lo, odd, surface)
-                    except CPRBoundaryStraddleError:
-                        got = "straddle"
-                    except CPRNoPositionError:
-                        got = "nopos"
-                    if isinstance(want, str):
-                        assert got == want, (surface, i, odd, got, want)
-                        straddle += want == "straddle"
-                        nopos += want == "nopos"
-                    else:
-                        assert got[0] == want[0] and got[1] == want[1], (surface, i, odd, got, want)     # lat/lon bit-exact
-                        assert abs(got[2] - want[2]) <= 1e-12 * max(1, want[2]) and abs(got[3] - want[3]) <= 1e-10
-                        ok += 1
-        assert ok > 2500 and nopos >= 2 * rounds and straddle > 0
-    finally:
-        mg.unload_reference()
+    stored = load_decode_ref_golden()["cpr_class"]
+    clock = mg.Clock()
+    ok = straddle = nopos = 0
+    for surface, (loc, events) in dc.cpr_class_script().items():
+        ours = decode.cpr_decoder(list(loc), clock=clock.time, _backend=_ShimBackend(shim, list(loc)))
+        wants = iter(stored[str(surface)])
+        for ev in events:
+            if ev[0] == "loc":
+                ours.set_location(list(ev[1]))
+                continue
+            _, clock.now, icao, la, lo, odd = ev
+            want = next(wants)
+            try:
+                got = ours.decode(icao, la, lo, odd, surface)
+            except CPRBoundaryStraddleError:
+                got = "straddle"
+            except CPRNoPositionError:
+                got = "nopos"
+            if isinstance(want, str):
+                assert got == want, (surface, ev, got, want)
+                straddle += want == "straddle"
+                nopos += want == "nopos"
+            else:
+                assert got[0] == want[0] and got[1] == want[1], (surface, ev, got, want)     # lat/lon bit-exact
+                assert abs(got[2] - want[2]) <= 1e-12 * max(1, want[2]) and abs(got[3] - want[3]) <= 1e-10
+                ok += 1
+        assert next(wants, None) is None
+    assert ok > 2500 and nopos >= 2 * 1500 and straddle > 0

@@ -20,7 +20,8 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 def libs(tmp_path_factory):
     d = tmp_path_factory.mktemp("simt")
     emul, shim = str(d / "libdecode_emul.so"), str(d / "libdecode_shim.so")
-    flags = ["g++", "-std=c++17", "-O1", "-U_FORTIFY_SOURCE", "-ffp-contract=off", "-Wno-unknown-pragmas", "-shared", "-fPIC"]
+    flags = ["g++", "-std=c++17", "-O1", "-U_FORTIFY_SOURCE", "-ffp-contract=off", "-Wno-unknown-pragmas", "-shared", "-fPIC",
+             "-Wl,-Bsymbolic"]                                                   # see test_library_simt.py
     subprocess.run(flags + ["-o", emul, os.path.join(ROOT, "tests", "simt", "decode_emul.cc")], check=True)
     subprocess.run(flags + ["-o", shim, os.path.join(ROOT, "tests", "decode_host_shim.cc")], check=True)
     e, s = C.CDLL(emul), C.CDLL(shim)

@@ -20,7 +20,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 def emul(tmp_path_factory):
     out = str(tmp_path_factory.mktemp("ksimt") / "libkernels_emul.so")
     subprocess.run(["g++", "-std=c++17", "-O1", "-U_FORTIFY_SOURCE", "-ffp-contract=off", "-Wno-unknown-pragmas", "-Wno-psabi", "-shared", "-fPIC",
-                    "-o", out, os.path.join(ROOT, "tests", "simt", "kernels_emul.cc")], check=True)
+                    "-Wl,-Bsymbolic", "-o", out, os.path.join(ROOT, "tests", "simt", "kernels_emul.cc")], check=True)   # see test_library_simt.py
     lib = C.CDLL(out)
     lib.emul_preamble.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_float, C.c_float, C.c_int, C.c_int, C.c_void_p,
                                   C.c_void_p, C.c_int, C.c_void_p]

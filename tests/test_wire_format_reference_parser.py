@@ -1,65 +1,32 @@
 """SURVEY.md 8 row f2: the message strings we emit are consumed by the reference's UNMODIFIED parser
-(python/parse.py make_parser, :422-436). Runs only where /root/reference exists (this container); the reference
-files are imported in place behind a stub `air_modes` package, never copied."""
-import importlib.util
+(python/parse.py make_parser, :422-436). What the parser published for each message of tests/golden/golden.json is
+stored by tests/golden/make_decode_ref_golden.py (the reference files imported in place behind a stub `air_modes`
+package, never copied); the messages themselves are what the oracle port computes for the golden scenes."""
 import math
-import os
-import sys
-import types
 
-import pytest
+from oracle import cpu_oracle as co
 
-from helpers import load_golden
-
-REF = "/root/reference/python"
-pytestmark = pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not present")
+from helpers import load_decode_ref_golden, load_golden
 
 
-def _load(name, path):
-    spec = importlib.util.spec_from_file_location(name, path)
-    mod = importlib.util.module_from_spec(spec)
-    sys.modules[name] = mod
-    spec.loader.exec_module(mod)
-    return mod
-
-
-@pytest.fixture()
-def ref_parser():
-    saved = {k: v for k, v in sys.modules.items() if k == "air_modes" or k.startswith("air_modes.")}
-    pkg = types.ModuleType("air_modes")
-    pkg.__path__ = []
-    sys.modules["air_modes"] = pkg
-    try:
-        _load("air_modes.exceptions", os.path.join(REF, "exceptions.py"))
-        _load("air_modes.altitude", os.path.join(REF, "altitude.py"))
-        mt = _load("air_modes.modes_types", os.path.join(REF, "modes_types.py"))
-        pkg.modes_report, pkg.stamp = mt.modes_report, mt.stamp
-        yield _load("air_modes.parse", os.path.join(REF, "parse.py"))
-    finally:
-        for k in [k for k in sys.modules if k == "air_modes" or k.startswith("air_modes.")]:
-            del sys.modules[k]
-        sys.modules.update(saved)
-
-
-def test_reference_parser_accepts_our_messages(ref_parser):
+def test_reference_parser_accepts_our_messages(port):
     meta, scenes = load_golden()
+    parsed = load_decode_ref_golden()["parser"]
     seen = 0
-    for s, _ in scenes:
-        pub = {}
-        publish = ref_parser.make_parser(pub)
-        for m in s["msgs"]:
-            pub.clear()
-            publish(m)
+    for s, iq in scenes:
+        msgs = port.run_iq(iq, s["rate"], s["threshold_db"], s["use_pmf"], co.MA_CANONICAL).msgs
+        assert msgs == s["msgs"], s["name"]
+        for m in msgs:
+            rep = parsed[m]
             data, ecc, ref, secs, frac = m.split()
-            if "modes_dl" not in pub:       # the parser drops types it has no handler for (ADSBError)
+            if rep is None:                 # the parser drops types it has no handler for (ADSBError)
                 continue
-            rep = pub["modes_dl"]
-            assert rep.ecc == int(ecc, 16)
-            assert abs(rep.rssi - 10.0 * math.log10(max(1e-8, float(ref)))) < 1e-12
-            assert rep.timestamp.secs == int(secs) and rep.timestamp.frac_secs == float(frac)
+            assert rep["ecc"] == int(ecc, 16)
+            assert abs(rep["rssi"] - 10.0 * math.log10(max(1e-8, float(ref)))) < 1e-12
+            assert rep["secs"] == int(secs) and rep["frac_secs"] == float(frac)
             df = int(data[:2], 16) >> 3
-            assert rep.data.get_type() == df and ("type%i_dl" % df) in pub
+            assert rep["df"] == df and rep["typed"]
             if df in (11, 17) and data in s["sent"]:
-                assert rep.data["aa"] == int(data[2:8], 16)      # ICAO address straight from our payload
+                assert rep["aa"] == int(data[2:8], 16)      # ICAO address straight from our payload
                 seen += 1
     assert seen >= 20
